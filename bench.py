@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W                 # our arm (one process per GPU via torchrun for N>1)
     python bench.py --impl reference --gpus N --steps K --warmup W  # the reference itself on the host CPU (baseline/_ref), rank 0 only
+    python bench.py --steps K --dump-outputs DIR                  # also write what the last timed step computed, as .npy
 
 A "step" is one full training step of the MAGVIT2 VideoTokenizer (GAN / perceptual terms disabled — the
 only configuration in which the reference runs offline, SURVEY.md §8) on one synthetic batch of
@@ -253,6 +254,25 @@ def _hbm_bytes(name, a):
     return None
 
 
+DUMP_PER_PARAM = 4096      # values per parameter in params_sample.npy: 0.67 M of the 375 M parameters, 2.7 MB
+
+
+def dump_outputs(out_dir, loss, model):
+    """What the last timed step hands its caller: the loss, and the parameters the optimizer step left behind (a fixed,
+    seeded sample of DUMP_PER_PARAM values of each, in named_parameters() order). Both float32."""
+    import numpy as np
+    gen = torch.Generator().manual_seed(0)
+    parts = []
+    for _, p in model.named_parameters():
+        flat = p.detach().flatten()
+        if flat.numel() > DUMP_PER_PARAM:
+            flat = flat[torch.randint(flat.numel(), (DUMP_PER_PARAM,), generator=gen).to(flat.device)]
+        parts.append(flat.float().cpu())
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, 'loss.npy'), loss.detach().float().cpu().reshape(1).numpy())
+    np.save(os.path.join(out_dir, 'params_sample.npy'), torch.cat(parts).numpy())
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
@@ -265,7 +285,11 @@ def main():
                     help='--impl reference: drop to 1 clip per step if (steps+warmup) x first-step time exceeds this')
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-graph', action='store_true', help='launch every kernel from Python instead of replaying the captured step')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write the loss and a sample of the updated parameters of the last one')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     rank, world, local = env_int('RANK', 0), env_int('WORLD_SIZE', 1), env_int('LOCAL_RANK', 0)
 
     if args.impl == 'reference':
@@ -362,10 +386,10 @@ def main():
         barrier()
         e0.record()
         for _ in range(args.steps):
-            fn()
+            out = fn()
         e1.record()
         barrier()
-        return max_over_ranks(e0.elapsed_time(e1))
+        return max_over_ranks(e0.elapsed_time(e1)), out
 
     def e2e_step():
         if use_graph:
@@ -377,15 +401,17 @@ def main():
     # ---------------- timed legs: e2e (a) -> device-resident `value` -> e2e (b) ----------------
     # The e2e leg brackets the value leg on both sides so that slow clock drift under the power cap cancels in the
     # comparison of the two (round 1 ran them back to back and e2e came out 1 % FASTER than value).
-    ms_e2e_a = timed(e2e_step)
+    ms_e2e_a, _ = timed(e2e_step)
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
     launches0 = _lib.launch_count()
-    ms_total = timed(lambda: train_step(dev_video))
+    ms_total, last_loss = timed(lambda: train_step(dev_video))
     launches = _lib.launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
-    ms_e2e_b = timed(e2e_step)
+    if args.dump_outputs and rank == 0:      # before the next leg replays the step again
+        dump_outputs(args.dump_outputs, last_loss, model)
+    ms_e2e_b, _ = timed(e2e_step)
     ms_e2e = 0.5 * (ms_e2e_a + ms_e2e_b)
 
     # ---------------- per-kernel timing pass (eager, CUDA events around every launch of the library) ----------

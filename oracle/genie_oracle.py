@@ -68,6 +68,13 @@ def det_indices(key: str, numel: int, n: int = 1024) -> Tensor:
     return ((u.double() + 1.0) * 0.5 * numel).long().clamp_(0, numel - 1)
 
 
+def det_sample(t: Tensor, key: str, n: int = 1024) -> Tensor:
+    """The flattened values of `t` at det_indices(key, t.numel(), n): how the goldens store big tensors. A stored
+    sample of m values is matched by det_sample(got, key, m), whether or not it holds the whole tensor."""
+    flat = t.detach().flatten()
+    return flat[det_indices(key, flat.numel(), n).to(flat.device)]
+
+
 def det_state_dict(shapes: Dict[str, Sequence[int]], gain: float = 1.0) -> StateDict:
     """Deterministic weights for a reference-format state_dict (shapes from the reference module).
 

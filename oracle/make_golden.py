@@ -39,6 +39,7 @@ from genie.dynamics import DynamicsModel                        # noqa: E402
 OUT = os.path.join(ROOT, 'tests', 'golden')
 os.makedirs(OUT, exist_ok=True)
 torch.set_num_threads(os.cpu_count())
+OUT_SAMPLE = 16384     # values stored per layer output / input gradient: keeps each golden file under 1 MB
 
 
 class ZeroLoss(nn.Module):
@@ -69,6 +70,12 @@ def close(a, b, name, rtol=1e-4, atol=1e-5):
 
 def grads_of(module):
     return {k: p.grad.detach().clone() for k, p in module.named_parameters() if p.grad is not None}
+
+
+def output_entry(key, y, dx, module):
+    """Output and input gradient of a layer as OUT_SAMPLE values each (det_sample), its gradients summarized."""
+    return {'y': O.det_sample(y, key + '.y', OUT_SAMPLE), 'dx': O.det_sample(dx, key + '.dx', OUT_SAMPLE),
+            'grads': summarize_grads(grads_of(module))}
 
 
 def summarize_grads(g, keep_full=()):
@@ -117,35 +124,35 @@ def gen_layers():
     sd = load_det(m)
     y = m(x); y.square().mean().backward()
     close(O.causal_conv3d(x, sd['conv3d.weight'], sd['conv3d.bias']), y, 'CausalConv3d k3')
-    out['causal_conv3d'] = {'y': y.detach(), 'dx': x.grad.clone(), 'grads': summarize_grads(grads_of(m))}
+    out['causal_conv3d'] = output_entry('layers.causal_conv3d', y, x.grad, m)
     x.grad = None
 
     m = SpaceTimeDownsample(64, 3, 64, time_factor=2, space_factor=2)
     sd = load_det(m)
     y = m(x); y.square().mean().backward()
     close(O.spacetime_downsample(sd, '', x, 2, 2), y, 'SpaceTimeDownsample')
-    out['spacetime_downsample'] = {'y': y.detach(), 'dx': x.grad.clone(), 'grads': summarize_grads(grads_of(m))}
+    out['spacetime_downsample'] = output_entry('layers.spacetime_downsample', y, x.grad, m)
     x.grad = None
 
     m = VideoResidualBlock(64, 128)
     sd = load_det(m)
     y = m(x); y.square().mean().backward()
     close(O.video_residual_block(sd, '', x), y, 'VideoResidualBlock 64->128')
-    out['video_residual'] = {'y': y.detach(), 'dx': x.grad.clone(), 'grads': summarize_grads(grads_of(m))}
+    out['video_residual'] = output_entry('layers.video_residual', y, x.grad, m)
     x.grad = None
 
     m = VideoResidualBlock(64, 128, downsample=(2, 2))      # blur-pool variant (README / test blueprints)
     sd = load_det(m)
     y = m(x); y.square().mean().backward()
     close(O.video_residual_block(sd, '', x, downsample=(2, 2)), y, 'VideoResidualBlock downsample')
-    out['video_residual_down'] = {'y': y.detach(), 'dx': x.grad.clone(), 'grads': summarize_grads(grads_of(m))}
+    out['video_residual_down'] = output_entry('layers.video_residual_down', y, x.grad, m)
     x.grad = None
 
     m = DepthToSpaceTimeUpsample(64, kernel_size=3, time_factor=2, space_factor=2)
     sd = load_det(m)
     y = m(x); y.square().mean().backward()
     close(O.depth2spacetime_upsample(sd, '', x, 2, 2), y, 'DepthToSpaceTimeUpsample')
-    out['depth2spacetime_upsample'] = {'y': y.detach(), 'dx': x.grad.clone(), 'grads': summarize_grads(grads_of(m))}
+    out['depth2spacetime_upsample'] = output_entry('layers.depth2spacetime_upsample', y, x.grad, m)
     x.grad = None
 
     m = AdaptiveGroupNorm(6, 8, 64)
@@ -153,7 +160,7 @@ def gen_layers():
     cond = O.det_uniform('layers.cond', (2, 6, 2, 4, 4)).sign()
     y = m(x, cond); y.square().mean().backward()
     close(O.adaptive_group_norm(sd, '', x, cond, 8), y, 'AdaptiveGroupNorm')
-    out['adaptive_group_norm'] = {'y': y.detach(), 'dx': x.grad.clone(), 'grads': summarize_grads(grads_of(m))}
+    out['adaptive_group_norm'] = output_entry('layers.adaptive_group_norm', y, x.grad, m)
     x.grad = None
     torch.save(out, os.path.join(OUT, 'layers.pt'))
 
@@ -188,7 +195,7 @@ def gen_st_block():
         y.square().mean().backward()
         oy = O.spacetime_attention(sd, '', x, 2, transpose, cond)
         close(oy, y, f'SpaceTimeAttention {tag}', rtol=2e-4, atol=2e-5)
-        out[tag] = {'y': y.detach(), 'dx': x.grad.clone(), 'grads': summarize_grads(grads_of(m))}
+        out[tag] = output_entry(f'st_block.{tag}', y, x.grad, m)
         x.grad = None
     torch.save(out, os.path.join(OUT, 'st_block.pt'))
 
@@ -381,10 +388,40 @@ def gen_generate():
     torch.save(out, os.path.join(OUT, 'generate.pt'))
 
 
+PLATFORMER_SAMPLE = 8192
+
+
+def gen_platformer():
+    """The reference's Platformer2D on the clips of fixtures.write_platformer_clips: for every output format and padding,
+    each clip's shape and a det_sample of its values, stored x 255 as uint8 (the frames are uint8 / 255, so exactly)."""
+    import shutil
+    import tempfile
+    from genie.module.data import Platformer2D
+    root = tempfile.mkdtemp(prefix='platformer_')
+    try:
+        fx.write_platformer_clips(root)
+        out = {}
+        for fmt in ('t c h w', 'c t h w'):
+            for padding in ('none', 'repeat', 'zero'):
+                ds = Platformer2D(root, split='train', padding=padding, num_frames=16, output_format=fmt)
+                for i, f in enumerate(ds.file_names):
+                    name = os.path.basename(f)
+                    v = O.det_sample(ds[i], f'platformer.{fmt}.{padding}.{name}', PLATFORMER_SAMPLE)
+                    u8 = (v * 255.).round().to(torch.uint8)
+                    assert torch.equal(u8.float() / 255., v)
+                    out[(fmt, padding, name)] = {'shape': tuple(ds[i].shape), 'x255': u8}
+    finally:
+        shutil.rmtree(root)
+    torch.save(out, os.path.join(OUT, 'platformer.pt'))
+
+
 if __name__ == '__main__':
     if sys.argv[1:] == ['generate']:
         with torch.no_grad():
             gen_generate()
+        sys.exit(0)
+    if sys.argv[1:] == ['platformer']:
+        gen_platformer()
         sys.exit(0)
     if sys.argv[1:] == ['gan']:
         gen_gan_perceptual()
@@ -399,5 +436,6 @@ if __name__ == '__main__':
     gen_st_block()
     gen_tokenizer()
     gen_action_dynamics()
+    gen_platformer()
     sizes = {f: os.path.getsize(os.path.join(OUT, f)) for f in sorted(os.listdir(OUT))}
     print('golden files:', sizes, 'total', sum(sizes.values()))

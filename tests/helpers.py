@@ -13,6 +13,11 @@ def det_weights(module, gain=1.0):
     return {k: v.detach().clone().cpu() for k, v in module.state_dict().items()}
 
 
+def at_sample(t, key, ref):
+    """`t` (reference layout) on the deterministic sample that the golden `ref` stores (genie_oracle.det_sample)."""
+    return O.det_sample(t.detach().float(), key, ref.numel()).cpu()
+
+
 def bf16_round(t):
     return t.to(torch.bfloat16).to(torch.float32)
 

@@ -1,50 +1,26 @@
-"""Data path (SURVEY.md §8 f4): Platformer2D / LightningPlatformer2D against the reference's own classes on mp4 files
-written here with OpenCV (CPU), and the device-side frame decode + prefetcher (GPU)."""
+"""Data path (SURVEY.md §8 f4): Platformer2D / LightningPlatformer2D on mp4 files written here with OpenCV (CPU),
+against what the reference's own Platformer2D returned for the same files (tests/golden/platformer.pt, written by
+oracle/make_golden.py), and the device-side frame decode + prefetcher (GPU)."""
 import os
-import sys
 
-import numpy as np
 import pytest
 import torch
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+from oracle import fixtures as fx
+from oracle import genie_oracle as O
 
 
 @pytest.fixture(scope='module')
 def clips(tmp_path_factory):
-    cv2 = pytest.importorskip('cv2')
+    pytest.importorskip('cv2')
     root = tmp_path_factory.mktemp('platformer')
-    rng = np.random.default_rng(0)
-    for split, n in (('train', 5), ('val', 2), ('test', 2)):
-        d = root / 'Coinrun' / split
-        d.mkdir(parents=True)
-        for i in range(n):
-            w = cv2.VideoWriter(str(d / f'clip{i}.mp4'), cv2.VideoWriter_fourcc(*'mp4v'), 15, (64, 64))
-            assert w.isOpened()
-            base = rng.integers(0, 255, (8, 8, 3))
-            for t in range(12 if i == 0 else 20):          # clip0 is SHORTER than num_frames = 16
-                frame = np.kron((base + 9 * t) % 256, np.ones((8, 8, 1))).astype(np.uint8)
-                w.write(frame)
-            w.release()
+    fx.write_platformer_clips(str(root))
     return str(root)
 
 
-def _reference_classes():
-    """The reference's own dataset classes, when the reference is reachable (build container / vendored copy)."""
-    for cand in ('/root/reference', os.path.join(ROOT, 'baseline', '_ref')):
-        if os.path.isdir(os.path.join(cand, 'genie')):
-            for p in (os.path.join(ROOT, 'oracle', '_shim'), cand):
-                if p not in sys.path:
-                    sys.path.insert(0, p)
-            from genie.module.data import Platformer2D            # noqa
-            from genie.dataset import LightningPlatformer2D       # noqa
-            return Platformer2D, LightningPlatformer2D
-    return None, None
-
-
-def test_platformer2d_matches_the_reference_dataset(clips):
+def test_platformer2d_matches_the_reference_dataset(clips, golden):
     import open_genie_b200 as og
-    RefP, RefL = _reference_classes()
+    ref = golden('platformer.pt')
     for fmt in ('t c h w', 'c t h w'):
         for padding in ('none', 'repeat', 'zero'):
             ds = og.Platformer2D(clips, split='train', padding=padding, num_frames=16, output_format=fmt)
@@ -54,11 +30,13 @@ def test_platformer2d_matches_the_reference_dataset(clips):
             assert v.shape == shape and v.dtype == torch.float32 and 0.0 <= float(v.min()) and float(v.max()) <= 1.0
             short = [ds[i] for i in range(5) if ds.file_names[i].endswith('clip0.mp4')][0]
             assert short.shape[0 if fmt == 't c h w' else 1] == 12        # whole (shorter) video: data.py:191-193
-            if RefP is not None:
-                rds = RefP(clips, split='train', padding=padding, num_frames=16, output_format=fmt)
-                assert rds.file_names == ds.file_names
-                for i in range(len(ds)):
-                    assert torch.equal(ds[i], rds[i])                          # bit-identical CPU tensors
+            root = os.path.join(clips, 'Coinrun', 'train')
+            assert ds.file_names == [os.path.join(root, f) for f in os.listdir(root)]     # data.py:163-166
+            for i, f in enumerate(ds.file_names):
+                key = (fmt, padding, os.path.basename(f))
+                want = ref[key]['x255'].float() / 255.                                 # exactly the reference's values
+                assert tuple(ds[i].shape) == ref[key]['shape']
+                assert torch.equal(O.det_sample(ds[i], 'platformer.{}.{}.{}'.format(*key), want.numel()), want)
     raw = og.Platformer2D(clips, split='val', num_frames=16, raw_uint8=True)[0]
     assert raw.dtype == torch.uint8 and raw.shape == (16, 64, 64, 3)
     ref = og.Platformer2D(clips, split='val', num_frames=16, output_format='t h w c')[0]

@@ -3,7 +3,7 @@ import pytest
 import torch
 import torch.nn.functional as F
 
-from helpers import assert_close, bf16_round, det_weights, rel_l2
+from helpers import assert_close, at_sample, bf16_round, det_weights, rel_l2
 from oracle import fixtures as fx
 from oracle import genie_oracle as O
 
@@ -182,11 +182,11 @@ def test_spacetime_attention_block_against_reference_golden(golden, case):
     t = shape[2] if transpose else shape[1]
     cond = O.det_uniform('st.cond', (2, t, 4)).sign().to(DEV) if cond_dim else None
     y = m(x, cond=(None, cond)) if cond_dim else m(x)
-    assert tuple(y.shape) == tuple(g['y'].shape)
+    assert tuple(y.shape) == tuple(shape)
     gy = (2.0 / y.numel()) * y.detach().float()
     y.backward(gy.to(y.dtype))
-    assert rel_l2(y.float().cpu(), g['y']) < 2e-2
-    assert rel_l2(x.grad.float().cpu(), g['dx']) < 6e-2
+    assert rel_l2(at_sample(y, f'st_block.{tag}.y', g['y']), g['y']) < 2e-2
+    assert rel_l2(at_sample(x.grad, f'st_block.{tag}.dx', g['dx']), g['dx']) < 6e-2
     grads = {k: p.grad.float().cpu() for k, p in m.named_parameters() if p.grad is not None}
     assert set(grads) == set(g['grads']['norm'])
     for k, v in g['grads']['full'].items():
